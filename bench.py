@@ -15,6 +15,8 @@ sweep 1..32.  N > 1 shards images across ranks (weak scaling, no data-path colle
 output latents per step.  Prints one JSON line on rank 0.
 
   --model/--stochastic/--batch/--dtype pick another headline workload; --configs none|3,4,5 limits the extra block.
+  --dump-outputs DIR writes what the headline step returned in its last timed step (DIR/image.npy, DIR/latent.npy, float32) so
+  that two builds can be compared output for output: the inputs and weights are seeded, identical from run to run.
 """
 import argparse
 import json
@@ -39,6 +41,7 @@ WORKLOADS = {
     "5": "cyclegan-turbo clear_to_rainy (a2b) fp16 512x512, per-GPU batch sweep (BASELINE config #5)",
 }
 WORKLOAD = WORKLOADS["2"]
+DUMP_BYTES = 60 << 20               # --dump-outputs budget over all arrays (< 64 MB)
 
 
 def measured_peaks():
@@ -108,6 +111,21 @@ def synthetic_inputs(B, size, cross_dim, dtype, device, seed_offset=0, kind="edg
     noise = torch.randn(B, 4, size // 8, size // 8, generator=torch.Generator().manual_seed(42 + seed_offset))
     mv = (lambda t: t.to(dtype).to(device)) if device else (lambda t: t.to(dtype))
     return mv(c_t), mv(text), mv(eps), mv(noise)
+
+
+def dump_outputs(d, arrays):
+    """Write each array as d/<name>.npy in float32.  When all of them together exceed DUMP_BYTES, each is reduced to a fixed,
+    seeded sample of its flattened elements (the same indices on every run of the same arguments)."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    total = sum(t.numel() * 4 for t in arrays.values())
+    for name, t in arrays.items():
+        a = t.detach().float().cpu()
+        if total > DUMP_BYTES:
+            n = a.numel() * DUMP_BYTES // total
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:n].sort().values
+            a = a.flatten()[idx]
+        np.save(os.path.join(d, name + ".npy"), a.numpy())
 
 
 def cpu_oracle_images_per_s(sd, size, steps, warmup, cross_dim, cfg):
@@ -313,7 +331,11 @@ def main():
     ap.add_argument("--configs", default="3,4,5", help="extra BASELINE configs reported in the `configs` block ('none' to skip)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-out", default="", help="write the per-launch timing table (JSON) here")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write rank 0's image and latent of the last timed headline step to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -364,6 +386,8 @@ def main():
         finish()
     ms_step, ms_mine = timed(step, K, 0, world, dist, flush, finish)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"image": wl.out, "latent": wl.lat})
     value = world * B / (ms_step / 1e3)
     finite = bool(torch.isfinite(wl.out.float()).all().item())
 
@@ -422,10 +446,9 @@ def main():
         call_u8 = lambda x: wl.model.forward_u8(x)
     e2e_u8_value = e2e_loop(lambda: u8_in.cuda(non_blocking=True), call_u8, lambda y: u8_out.copy_(y, non_blocking=True), gathered_u8)
 
-    # ---- the other BASELINE configs, same N, same timing rules (fewer steps) ----
+    # ---- the other BASELINE configs, same N, same timing rules ----
     configs = {head_id: {"workload": workload, "value": value, "ms_per_step": ms_step, "per_gpu_batch": B, "dtype": args.dtype,
                          "finite": finite}}
-    Kx = max(3, min(K, 5))
     cyc = None
     for cid in extra:
         try:
@@ -442,14 +465,14 @@ def main():
             for b in sweep:
                 w2.set_batch(b)
                 step2, fin2, _ = make_step(w2, world, dist)
-                ms2, _ = timed(step2, Kx, 3, world, dist, flush, fin2)
+                ms2, _ = timed(step2, K, 3, world, dist, flush, fin2)
                 if fin2 is not None:
                     fin2()
                     torch.cuda.synchronize()
                 rows.append({"per_gpu_batch": b, "global_batch": world * b, "value": world * b / (ms2 / 1e3), "ms_per_step": ms2,
                              "finite": bool(torch.isfinite(w2.out.float()).all().item()),
                              "step_tensor_frac_of_sustained_peak": (b * FLOPS_PER_IMAGE / (ms2 * 1e-3)) / 1e12 / measured_peaks()[0]})
-            entry = {"workload": WORKLOADS[cid], "dtype": "fp16" if w2.dt == torch.float16 else "bf16", "steps": Kx, "warmup": 3,
+            entry = {"workload": WORKLOADS[cid], "dtype": "fp16" if w2.dt == torch.float16 else "bf16", "steps": K, "warmup": 3,
                      "n_gpus": world}
             if cid == "5":
                 entry["sweep"] = rows

@@ -1,8 +1,8 @@
-"""TEST DOUBLE of i2it.Engine for GPU-less hosts — test infrastructure, never imported by the product.
+"""TEST DOUBLE of i2it.Engine that computes on the CPU — test infrastructure, never imported by the product.
 
-Purpose: run the UNMODIFIED reference CLIs (/root/reference/src/inference_paired.py, inference_unpaired.py) in this container
-(no GPU) against the repo's drop-in modules (pix2pix_turbo / cyclegan_turbo / model), to prove the import contract and the call
-sequence of SURVEY.md section 8b end to end: constructor kwargs, .set_eval()/.eval()/.half(),
+Purpose: run the reference's inference CLIs (src/inference_paired.py, inference_unpaired.py: live when recording, replayed from
+tests/golden/ in the suite) on any host against the repo's drop-in modules (pix2pix_turbo / cyclegan_turbo / model), to prove
+the import contract and the call sequence of SURVEY.md section 8b end to end: constructor kwargs, .set_eval()/.eval()/.half(),
 .unet.enable_xformers_memory_efficient_attention(), forward signatures, dtype/shape of what comes back.
 
 The stub implements the i2it.Engine methods the wrappers call and computes with the CPU ORACLE (tests may import oracle/), so the

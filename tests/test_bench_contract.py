@@ -1,10 +1,13 @@
-"""CPU checks of the bench.py contract that do not need a GPU: the reference arm (the oracle timed on the host cores) prints one
+"""Checks of the bench.py contract.  Without a GPU: the reference arm (the oracle timed on the host cores) prints one
 well-formed JSON line, non-zero ranks of a torchrun launch stay silent and exit 0, and the product arm refuses to run without
-a CUDA device instead of falling back to anything."""
+a CUDA device instead of falling back to anything.  On the GPU: --dump-outputs writes reproducible outputs."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -42,3 +45,41 @@ def test_product_arm_needs_a_gpu():
         return
     r = _run(["--steps", "1", "--warmup", "1"], timeout=300)
     assert r.returncode != 0 and "{" not in r.stdout          # no number is printed, nothing falls back to the CPU
+
+
+def test_dump_outputs_over_budget_keep_one_seeded_sample(tmp_path, monkeypatch):
+    """Outputs larger than the dump budget are cut to the same seeded sample of their elements on every call, within budget."""
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4096)
+    outs = {"image": torch.randn(2, 3, 32, 32, dtype=torch.bfloat16), "latent": torch.randn(2, 4, 4, 4, dtype=torch.bfloat16)}
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), outs)
+    got = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in outs}
+    assert sum(a.nbytes for a in got.values()) <= 4096
+    for n, t in outs.items():
+        assert got[n].dtype == np.float32 and got[n].size > 0
+        assert np.array_equal(got[n], np.load(tmp_path / "b" / f"{n}.npy"))
+        assert np.isin(got[n], t.float().numpy().ravel()).all()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_repeat_bit_for_bit(tmp_path):
+    """--dump-outputs writes the last timed step's image and latent as float32 .npy; --steps sets the timed step count; two runs
+    with the same arguments get the same seeded inputs, so the dumps of one build agree bit for bit."""
+    dumps = []
+    for i in range(2):
+        d = tmp_path / f"run{i}"
+        r = _run(["--steps", "2", "--warmup", "1", "--batch", "1", "--configs", "none", "--no-cpu-baseline",
+                  "--dump-outputs", str(d)], timeout=900)
+        assert r.returncode == 0, r.stderr[-3000:]
+        line = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+        assert line["steps"] == 2 and line["finite"]
+        assert sorted(os.listdir(d)) == ["image.npy", "latent.npy"]
+        a = {n: np.load(d / f"{n}.npy") for n in ("image", "latent")}
+        assert a["image"].shape == (1, 3, 512, 512) and a["latent"].shape == (1, 4, 64, 64)
+        assert all(v.dtype == np.float32 and np.isfinite(v).all() for v in a.values())
+        dumps.append(a)
+    for n in dumps[0]:
+        assert np.array_equal(dumps[0][n], dumps[1][n]), n

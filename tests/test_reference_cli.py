@@ -1,93 +1,69 @@
-"""The UNMODIFIED reference CLIs run against the drop-in modules (VERDICT r1 missing #7; SURVEY.md section 8b "call it unchanged").
+"""The reference's UNMODIFIED inference CLIs against the drop-in modules (VERDICT r1 missing #7; SURVEY.md section 8b "call it
+unchanged"), replayed from golden recordings.
 
-/root/reference exists only in the build container (not on the GPU box), and the container has no GPU: so these are CPU tests,
-skipped when the reference tree is absent.  The engine is replaced by tests/cpu_stub_engine.py (a test double computing with the
-CPU oracle); everything else — module resolution, constructor/forward/half/eval calls, checkpoint reading, PIL in / PIL out — is
-the real host code of this repo driven by the reference's own script."""
-import json
+tests/golden/reference_cli_*.pt hold what src/inference_paired.py and src/inference_unpaired.py did with this repo's modules when
+they were run (`python tests/run_reference_cli.py record <reference>/src`): the constructor arguments, each call on the model in
+order with its arguments and RNG state, the tensors that came back and the calls the engine received.  The test replays those
+calls on the current code and requires the same call sequence to be accepted and the same results to come back.  The engine is
+the CPU test double (tests/cpu_stub_engine.py, the CPU oracle) in both; everything else — module resolution, constructor /
+forward / half / eval calls, checkpoint reading — is the real host code of this repo."""
 import os
 import subprocess
 import sys
 
-import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/src"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
 
 
-def _run(script, args, cwd, timeout=900):
+def _replay(case, tmp_path, timeout=900):
     env = dict(os.environ)
     env["PYTHONPATH"] = ""
     env["I2IT_CFG"] = "tiny"        # the CLI cannot pass a reduced config: the drop-in modules take it from the environment
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "run_reference_cli.py"), os.path.join(REF, script)] + args,
-                       capture_output=True, text=True, cwd=cwd, env=env, timeout=timeout)
+    out = tmp_path / "replay.pt"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "run_reference_cli.py"), "replay", case, str(out)],
+                       capture_output=True, text=True, env=env, timeout=timeout)
     assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
-    return r.stdout
-
-
-def _png(path, w, h, seed):
-    from PIL import Image
-    g = torch.Generator().manual_seed(seed)
-    Image.fromarray((torch.rand(h, w, 3, generator=g) * 255).to(torch.uint8).numpy()).save(path)
+    gold = torch.load(os.path.join(ROOT, "tests", "golden", f"reference_cli_{case}.pt"))
+    got = torch.load(str(out))
+    assert len(got["results"]) == len(gold["calls"])
+    for c, r in zip(gold["calls"], got["results"]):
+        want = c["result"]
+        if isinstance(want, torch.Tensor):
+            assert isinstance(r, torch.Tensor) and r.shape == want.shape and r.dtype == want.dtype, (c["call"], r)
+            assert (r.float() - want.float()).abs().max() < 5e-3, c["call"]
+        else:
+            assert r == want, (c["call"], r, want)
+    assert got["engine_calls"] == gold["engine_calls"]
+    return gold, got
 
 
 def test_inference_paired_unmodified(tmp_path):
     """src/inference_paired.py --model_path <save_model() pickle> --use_fp16: reference lines 32-35 (ctor, set_eval, half),
     38-41 (crop to a multiple of 8), 66-72 (to_tensor, .cuda().half(), model(c_t, prompt), ToPILImage)."""
-    sys.path.insert(0, os.path.join(ROOT, "img2img-turbo_b200"))
-    import weights as W
-    from pix2pix_turbo import Pix2Pix_Turbo
-
-    class Tok:
-        model_max_length = 77
-    m = Pix2Pix_Turbo(cfg=W.TINY, text_stack=(Tok(), None), seed=3)   # reduced widths (I2IT_CFG=tiny on the CLI side): CPU minutes, not hours
-    ck = str(tmp_path / "model.pkl")
-    m.save_model(ck)
-    _png(str(tmp_path / "in.png"), 70, 66, 1)                     # 70x66 -> cropped to 64x64 by the script (multiples of 8)
-    out = _run("inference_paired.py", ["--input_image", str(tmp_path / "in.png"), "--prompt", "a test prompt", "--model_path", ck,
-                                      "--output_dir", str(tmp_path / "out"), "--use_fp16"], cwd=str(tmp_path))
-    from PIL import Image
-    img = Image.open(str(tmp_path / "out" / "in.png"))
-    assert img.size == (64, 64) and img.mode == "RGB"
-    assert os.path.join(ROOT, "img2img-turbo_b200", "pix2pix_turbo.py") in out        # the script imported OUR module
-    calls = json.loads(out.split("STUB_CALLS ", 1)[1].splitlines()[0])
-    kinds = [c[0] for c in calls]
+    gold, got = _replay("inference_paired", tmp_path)
+    assert gold["module"] == os.path.join("img2img-turbo_b200", "pix2pix_turbo.py")   # the script imported OUR module
+    assert [c["call"] for c in gold["calls"]] == ["__init__", "set_eval", "half", "__call__"]
+    assert gold["calls"][0]["kwargs"] == {"pretrained_name": "", "pretrained_path": "{model}"}
+    fwd_call = gold["calls"][-1]
+    assert fwd_call["args"][0].shape == (1, 3, 64, 64) and fwd_call["args"][1] == "a test prompt"   # 70x66 -> cropped to 64x64
+    assert gold["output_image"] == [64, 64, "RGB"]
+    kinds = [c[0] for c in got["engine_calls"]]
     assert kinds.count("forward") == 1 and "set_text" in kinds and "finalize" in kinds
-    fwd = next(c for c in calls if c[0] == "forward")
+    fwd = next(c for c in got["engine_calls"] if c[0] == "forward")
     assert fwd[1] == "(1, 3, 64, 64)" and fwd[2] == "torch.float16" and fwd[3] == "False"   # deterministic path, fp16
 
 
 def test_inference_unpaired_unmodified(tmp_path):
     """src/inference_unpaired.py --model_path <train_cyclegan_turbo.py-format pickle> --prompt ... --direction a2b --use_fp16:
     reference lines 34-38 (ctor, eval, enable_xformers..., half), 40-50 (build_transform, ToTensor, Normalize, model(x_t, ...))."""
-    sys.path.insert(0, os.path.join(ROOT, "img2img-turbo_b200"))
-    from cyclegan_turbo import CycleGAN_Turbo
-
-    class Tok:
-        model_max_length = 77
-    import weights as W
-    m = CycleGAN_Turbo(cfg=W.TINY, text_stack=(Tok(), None), synthetic_caption="c", synthetic_direction="a2b", seed=4)
-    # the checkpoint format written by train_cyclegan_turbo.py:293-307
-    def part(adapter):
-        return {k[len("unet."):].replace(f".{adapter}.weight", ".weight"): v for k, v in m._sd.items()
-                if k.startswith("unet.") and f".{adapter}." in k}
-    ck = {"rank_unet": 8, "rank_vae": 4, "l_target_modules_encoder": [], "l_target_modules_decoder": [], "l_modules_others": [],
-          "vae_lora_target_modules": [], "sd_encoder": part("default_encoder"), "sd_decoder": part("default_decoder"),
-          "sd_other": part("default_others"),
-          # (the real files carry the full VAE state dicts; the trained tensors — LoRA pairs and skip convs — are enough here)
-          "sd_vae_enc": {k: v for k, v in m._sd.items() if k.startswith(("vae.encoder", "vae_b2a.encoder")) and "lora" in k},
-          "sd_vae_dec": {k: v for k, v in m._sd.items() if k.startswith(("vae.decoder", "vae_b2a.decoder")) and ("lora" in k or "skip" in k)}}
-    p = str(tmp_path / "cyc.pkl")
-    torch.save(ck, p)
-    _png(str(tmp_path / "photo.png"), 128, 64, 2)
-    out = _run("inference_unpaired.py", ["--input_image", str(tmp_path / "photo.png"), "--prompt", "driving in the night",
-                                        "--model_path", p, "--direction", "a2b", "--output_dir", str(tmp_path / "out"),
-                                        "--image_prep", "no_resize", "--use_fp16"], cwd=str(tmp_path))
-    from PIL import Image
-    img = Image.open(str(tmp_path / "out" / "photo.png"))
-    assert img.size == (128, 64)                                   # resized back to the input size (reference :54)
-    calls = json.loads(out.split("STUB_CALLS ", 1)[1].splitlines()[0])
-    fwd = next(c for c in calls if c[0] == "forward")
+    gold, got = _replay("inference_unpaired", tmp_path)
+    assert gold["module"] == os.path.join("img2img-turbo_b200", "cyclegan_turbo.py")
+    assert [c["call"] for c in gold["calls"]] == ["__init__", "eval", "unet.enable_xformers_memory_efficient_attention", "half",
+                                                  "__call__"]
+    fwd_call = gold["calls"][-1]
+    assert fwd_call["args"][0].shape == (1, 3, 64, 128)
+    assert fwd_call["kwargs"] == {"direction": "a2b", "caption": "driving in the night"}
+    assert gold["output_image"][:2] == [128, 64]                   # resized back to the input size (reference :54)
+    fwd = next(c for c in got["engine_calls"] if c[0] == "forward")
     assert fwd[1] == "(1, 3, 64, 128)" and fwd[2] == "torch.float16" and fwd[5] == "0"       # a2b
