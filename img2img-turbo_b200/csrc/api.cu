@@ -1,5 +1,6 @@
 // extern "C" boundary of libi2it (see include/i2it.h).  Nothing throws across it.
 #include "engine.cuh"
+#include "canny.cuh"
 
 using namespace i2it;
 
@@ -136,6 +137,20 @@ int i2it_forward_u8(i2it_handle* h, const void* x_u8_hwc, int in_mode, const voi
   io.out_u8 = out_u8_hwc; io.out_latent = out_latent;
   E.check_device_error();
   E.forward(io, batch, H, W, direction, text_batch, static_cast<cudaStream_t>(stream));
+  API_END
+}
+
+int i2it_canny_u8(i2it_handle* h, const void* x_u8_hwc, int batch, int H, int W, float low_threshold, float high_threshold,
+                  void* out_u8_hwc, void* stream) {
+  API_BEGIN(h)
+  I2IT_CHECK(x_u8_hwc && out_u8_hwc, "i2it_canny_u8: null image pointer");
+  I2IT_CHECK(batch > 0 && H > 0 && W > 0, "i2it_canny_u8: batch, H and W must be positive");
+  const long long n = static_cast<long long>(batch) * H * W;
+  I2IT_CHECK(n < (1ll << 31), "i2it_canny_u8: batch*H*W must be below 2^31 (int32 labels)");
+  I2IT_CHECK(std::isfinite(low_threshold) && std::isfinite(high_threshold), "i2it_canny_u8: thresholds must be finite");
+  void* ws = E.canny_workspace(canny_workspace_bytes(n));
+  launch_canny(static_cast<const uint8_t*>(x_u8_hwc), batch, H, W, low_threshold, high_threshold,
+               static_cast<uint8_t*>(out_u8_hwc), ws, static_cast<cudaStream_t>(stream));
   API_END
 }
 

@@ -160,6 +160,7 @@ Engine::~Engine() {
   textenc_.clear();
   free_prepared();
   for (auto& kv : w_) cudaFree(kv.second.d);
+  if (canny_ws_) cudaFree(canny_ws_);
   if (err_host_) cudaFreeHost(err_host_);
   if (gstream_) cudaStreamDestroy(gstream_);
   if (ev_in_) cudaEventDestroy(ev_in_);
@@ -172,6 +173,17 @@ void Engine::check_device_error() {
     throw Error("tapgemm watchdog tripped (pipeline stage code " + std::to_string(code) +
                 ": 1=producer/empty 2=mma/tmem_empty 3=mma/full 4=epilogue/tmem_full)");
   }
+}
+
+void* Engine::canny_workspace(size_t bytes) {
+  if (bytes > canny_ws_bytes_) {
+    if (canny_ws_) I2IT_CUDA(cudaFree(canny_ws_));     // cudaFree waits for the device: no launch still uses the old buffer
+    canny_ws_ = nullptr;
+    canny_ws_bytes_ = 0;
+    I2IT_CUDA(cudaMalloc(&canny_ws_, bytes));
+    canny_ws_bytes_ = bytes;
+  }
+  return canny_ws_;
 }
 
 void* Engine::dmalloc(size_t bytes) {

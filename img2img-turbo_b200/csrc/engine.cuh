@@ -182,6 +182,7 @@ class Engine {
   void encode_text(const int* tokens, int batch, void* out, cudaStream_t st);
   bool has_text_encoder() const { return has("text_encoder.text_model.embeddings.token_embedding.weight"); }
   Plan* last_plan() const { return last_plan_; }
+  void* canny_workspace(size_t bytes);                            // i2it_canny_u8 scratch, grown on demand
   void read_stage(const std::string& name, float* dst, size_t dst_elems, int dims[4]);
 
   // ---- op builders (append launches to a plan) ----
@@ -280,6 +281,8 @@ class Engine {
   std::map<int, std::unique_ptr<Plan>> textenc_;            // CLIP text tower plans, by batch
   std::map<std::vector<int>, std::unique_ptr<Plan>> plans_;
   Plan* last_plan_ = nullptr;
+  void* canny_ws_ = nullptr;
+  size_t canny_ws_bytes_ = 0;
   Act text_;                     // staged text embedding while a UNet plan is being built
   TextKV* text_kv_ = nullptr;    // ... or the cached cross-attention operands (text_emb == NULL forwards)
 

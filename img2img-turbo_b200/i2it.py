@@ -29,7 +29,7 @@ SYMBOLS = [
     "i2it_default_config", "i2it_create", "i2it_destroy", "i2it_last_error", "i2it_set_weight",
     "i2it_set_adapter_scale", "i2it_finalize_weights", "i2it_workspace_bytes", "i2it_forward",
     "i2it_set_text", "i2it_encode_text", "i2it_forward_u8", "i2it_prep_launch_count", "i2it_debug_fast_div", "i2it_launch_count", "i2it_profile", "i2it_read_stage", "i2it_op_conv2d", "i2it_op_group_norm", "i2it_op_layer_norm",
-    "i2it_op_attention", "i2it_op_upsample2x",
+    "i2it_op_attention", "i2it_op_upsample2x", "i2it_canny_u8",
 ]
 
 
@@ -72,6 +72,7 @@ def load_library(path: Optional[str] = None):
     lib.i2it_set_text.argtypes = [vp, vp, ci, vp]
     lib.i2it_encode_text.argtypes = [vp, vp, ci, vp, vp]
     lib.i2it_forward_u8.argtypes = [vp, vp, ci, vp, ci, vp, vp, cf, vp, vp, ci, ci, ci, ci, vp]
+    lib.i2it_canny_u8.argtypes = [vp, vp, ci, ci, ci, cf, cf, vp, vp]
     lib.i2it_prep_launch_count.argtypes = [vp, C.POINTER(ci)]
     lib.i2it_debug_fast_div.argtypes = [C.c_longlong, ci, ci]
     lib.i2it_debug_fast_div.restype = C.c_longlong
@@ -229,6 +230,20 @@ class Engine:
         self._check(self.lib.i2it_forward_u8(self._h, _ptr(x_u8), int(in_mode), _ptr(text_emb), tb, _ptr(eps), _ptr(noise_map),
                                              float(r), _ptr(out), _ptr(out_latent), B, H, W, direction, _stream()),
                     "i2it_forward_u8")
+        return out
+
+    def canny_u8(self, x_u8: torch.Tensor, low: float, high: float, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """cv2.Canny(img, low, high) of every image, bit for bit, replicated to three channels: x_u8 [B,H,W,3] uint8 CUDA (RGB)
+        -> [B,H,W,3] uint8 CUDA in {0, 255}, ready for forward_u8(..., IN_UNIT, ...)."""
+        if not (x_u8.dtype == torch.uint8 and x_u8.is_cuda and x_u8.is_contiguous() and x_u8.dim() == 4 and x_u8.shape[3] == 3):
+            raise ValueError("canny_u8: image must be a contiguous uint8 CUDA tensor [B,H,W,3]")
+        if out is None:
+            out = torch.empty_like(x_u8)
+        if not (out.dtype == torch.uint8 and out.is_cuda and out.is_contiguous() and out.shape == x_u8.shape):
+            raise ValueError("canny_u8: out must be a contiguous uint8 CUDA tensor shaped like the image")
+        B, H, W, _ = x_u8.shape
+        self._check(self.lib.i2it_canny_u8(self._h, _ptr(x_u8), B, H, W, float(low), float(high), _ptr(out), _stream()),
+                    "i2it_canny_u8")
         return out
 
     def prep_launch_count(self) -> int:

@@ -221,3 +221,14 @@ class Pix2Pix_Turbo(TurboBase):
         if self._twin:
             self.unet.conv_in.r = None
         return out
+
+    def canny_u8(self, images_u8, low_threshold=100, high_threshold=200):
+        """Edge maps of photos on the device, bit for bit what the reference CLI feeds the model
+        (canny_from_pil, src/image_prep.py:6-12; default thresholds of src/inference_paired.py:18-19):
+        `images_u8` [B,H,W,3] (or [H,W,3]) uint8 RGB, host or device -> [B,H,W,3] uint8 CUDA tensor in {0, 255}.
+        Photo to image: `forward_u8(canny_u8(photo), prompt)`; the inverted map the CLI saves is `255 - edges`."""
+        x = torch.as_tensor(images_u8)
+        if x.dim() == 3:
+            x = x.unsqueeze(0)
+        x = x.to(device=_host.DEVICE, non_blocking=True).contiguous()
+        return self._get_engine().canny_u8(x, low_threshold, high_threshold)

@@ -129,6 +129,15 @@ int i2it_forward_u8(i2it_handle* h, const void* x_u8_hwc, int in_mode, const voi
                     const void* eps, const void* noise_map, float r, void* out_u8_hwc, void* out_latent, int batch,
                     int H, int W, int direction, void* stream);
 
+/* cv2.Canny(img, low_threshold, high_threshold) (apertureSize 3, L1 gradient) of each RGB image, replicated to three
+ * channels: np.array(canny_from_pil(img)) of the reference's src/image_prep.py:6-12, bit for bit.  x_u8_hwc, out_u8_hwc:
+ * [batch, H, W, 3] uint8 device pointers; any H, W >= 1 with batch*H*W < 2^31.  Values {0, 255}.  Thresholds are floored and
+ * ordered as cv2 does; non-finite ones are rejected.  Four launches enqueued on `stream` (not part of the forward's CUDA
+ * graph); needs no weights.  The workspace (6 bytes per pixel) is owned by the handle and grown on demand.  The output
+ * feeds i2it_forward_u8(..., I2IT_IN_UNIT, ...) as is. */
+int i2it_canny_u8(i2it_handle* h, const void* x_u8_hwc, int batch, int H, int W, float low_threshold,
+                  float high_threshold, void* out_u8_hwc, void* stream);
+
 /* Number of kernel launches one forward of this shape issues (for bench accounting): the plan the last forward used if it
  * has this shape, else the plan with the text embedding passed inline. */
 int i2it_launch_count(i2it_handle* h, int batch, int H, int W, int direction, int* launches);
