@@ -72,16 +72,6 @@ __device__ __forceinline__ float ex2_approx(float x) {
   return y;
 }
 __device__ __forceinline__ float silu_f(float x) { return __fdividef(x, 1.0f + ex2_approx(-1.4426950408889634f * x)); }
-// Programmatic dependent launch (PDL).  Every kernel of a forward plan calls pdl_sync() before its first access to global
-// memory: launch_dependents lets the NEXT kernel's CTAs become resident (and run their barrier/TMEM prologue) as soon as all
-// CTAs of this grid have started; wait blocks until the PREVIOUS grid has completed and its writes are visible.  Because
-// every kernel waits, completion is transitive along the stream (C waits for B, B waited for A), which keeps the pool's
-// buffer recycling safe.  Kernels that allocate TMEM call it AFTER the allocation, so an early-resident successor can never
-// take tensor memory a predecessor CTA still has to allocate.  Without the launch attribute both instructions are no-ops.
-__device__ __forceinline__ void pdl_sync() {
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-}
 
 // erf via Abramowitz-Stegun 7.1.26 (|abs err| < 1.5e-7, far below the 16-bit output rounding): 1 rcp + 1 ex2 + 7 FMA
 __device__ __forceinline__ float erf_as(float x) {

@@ -102,8 +102,6 @@ __global__ void cvt16_to_f32_kernel(const uint16_t* s, float* d, long long n, in
   else d[i] = __half2float(reinterpret_cast<const __half*>(s)[i]);
 }
 
-thread_local PdlState g_pdl;
-
 Engine::Engine(const i2it_config& c) : cfg(c), dtype(c.dtype) {
   I2IT_CHECK(c.dtype == DT_F16 || c.dtype == DT_BF16, "dtype must be I2IT_F16 or I2IT_BF16");
   I2IT_CUDA(cudaSetDevice(c.device));
@@ -118,26 +116,15 @@ Engine::Engine(const i2it_config& c) : cfg(c), dtype(c.dtype) {
   I2IT_CUDA(cudaFuncSetAttribute(tapgemm_kernel<__nv_bfloat16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TG_SMEM));
   I2IT_CUDA(cudaFuncSetAttribute(flash_attn_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize, FA_SMEM));
   I2IT_CUDA(cudaFuncSetAttribute(flash_attn_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, FA_SMEM));
-  I2IT_CUDA(cudaFuncSetAttribute(flash_attn_v1_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize, FA_SMEM));
-  I2IT_CUDA(cudaFuncSetAttribute(flash_attn_v1_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, FA_SMEM));
-  use_flash = std::getenv("I2IT_NO_FLASH") == nullptr;
-  flash_v1 = std::getenv("I2IT_FLASH_V1") != nullptr;       // round-1 softmax scheme (A/B)
   use_pair = std::getenv("I2IT_NO_PAIR") == nullptr;
-  use_pdl = std::getenv("I2IT_PDL") != nullptr;     // programmatic dependent launch: measured neutral (1 CTA/SM kernels cannot co-reside), opt-in
 #ifdef I2IT_TRACE_BUILD
   trace_on = std::getenv("I2IT_TRACE") != nullptr;
 #endif
   use_tmaout = std::getenv("I2IT_NO_TMAOUT") == nullptr;   // TMA-store epilogue (per-thread stores otherwise)
-  use_ostg2 = std::getenv("I2IT_NO_OSTG2") == nullptr;     // second TMA-store box per epilogue warp where the operand ring can spare 32 KB
   sync_each = std::getenv("I2IT_SYNC_EACH") != nullptr;    // eager path: synchronise after every launch and name the one that faults
   use_lean = std::getenv("I2IT_NO_LEAN") == nullptr;       // compile-time-stripped epilogue for the plain (no activation) TMA-store launches
   use_gnepi = std::getenv("I2IT_NO_GNEPI") == nullptr;     // GroupNorm statistics in the producing GEMM's epilogue
   use_splitk = std::getenv("I2IT_NO_SPLITK") == nullptr;   // split-K for the 8x8 1280-channel convs
-  use_catfuse = std::getenv("I2IT_NO_CATFUSE") == nullptr; // UNet skip concatenations written in place (no copy kernels)
-  pair_min_tiles = std::getenv("I2IT_PAIR_MIN_TILES") ? atoll(std::getenv("I2IT_PAIR_MIN_TILES")) : 2ll * num_sms;
-  // identity residual as a K-slab: round 1's default; with the round-2 epilogue (coalesced residual through the store box) and the
-  // faster halo path the residual is cheaper in the epilogue (9-tap halo conv 409 us vs 10-tap 585 us, run J), so it is opt-in now
-  use_idres = std::getenv("I2IT_IDRES") != nullptr && std::getenv("I2IT_NO_IDRES") == nullptr;
   use_halo = std::getenv("I2IT_NO_HALO") == nullptr;   // 3x3 convs: one halo tile per k-chunk instead of nine shifted A boxes
   I2IT_CUDA(cudaFuncSetAttribute(tapgemm2_kernel<__half, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TG2_SMEM));
   I2IT_CUDA(cudaFuncSetAttribute(tapgemm2_kernel<__half, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TG2_SMEM));
@@ -419,21 +406,6 @@ PW Engine::prep_im2col3(const std::string& name) {
   return pw;
 }
 
-PW Engine::prep_identity(int n) {
-  const std::string key = "identity|" + std::to_string(n);
-  auto it = prepared_.find(key);
-  if (it != prepared_.end()) return it->second;
-  PW pw;
-  pw.rows = n; pw.cin = n; pw.cin_pad = n; pw.taps = 1;
-  pw.w = static_cast<uint16_t*>(dmalloc(static_cast<size_t>(n) * n * 2));
-  PrepJob j;
-  std::memset(&j, 0, sizeof j);
-  j.mode = PREP_IDENTITY; j.out = pw.w; j.cout = n; j.n = static_cast<long long>(n) * n;
-  push_job(j);
-  prepared_[key] = pw;
-  return pw;
-}
-
 PW Engine::prep_subpixel(const std::string& name) {
   const std::string key = name + "|subpixel";
   auto it = prepared_.find(key);
@@ -600,7 +572,7 @@ void Engine::launch_gemm(Plan& P, const TmapSpec& sa, TmapSpec sb, const TapGemm
   const long long total_tiles = m_tiles * p.n_tiles * (p.ksplit > 1 ? p.ksplit : 1);
   // CTA-pair kernel: weights/B shared by every M tile (no per-tile B batch coordinates), enough tiles to fill the chip twice
   const bool pair = use_pair && p.ksplit <= 1 && p.b_mul[0] == 0 && p.b_mul[1] == 0 && p.b_mul[2] == 0 && (p.BN % 32) == 0 &&
-                    total_tiles >= pair_min_tiles && m_tiles >= 2;
+                    total_tiles >= 2ll * num_sms && m_tiles >= 2;
   TmapSpec sb2 = sb2p ? *sb2p : sb;
   if (pair) { sb.box[1] = p.BN / 2; sb2.box[1] = p.BN / 2; p.idesc = make_idesc2(dtype, p.BN); }
   p.halo = (pair && shalo != nullptr && use_halo) ? 1 : 0;
@@ -608,15 +580,8 @@ void Engine::launch_gemm(Plan& P, const TmapSpec& sa, TmapSpec sb, const TapGemm
   {  // smem ring geometry: B stage = the real (half) tile rounded to the 1024-byte swizzle atom, as many stages as fit
     const int brows = pair ? p.BN / 2 : p.BN;
     p.b_stage = (brows * TG_BK * 2 + 1023) / 1024 * 1024;
-    int budget = pair ? (p.halo ? TG2_DATA_BYTES - TG2_HALO_REGION : TG2_DATA_BYTES) : TG_STAGES * (TG_A_STAGE + TG_B_STAGE);
+    const int budget = pair ? (p.halo ? TG2_DATA_BYTES - TG2_HALO_REGION : TG2_DATA_BYTES) : TG_STAGES * (TG_A_STAGE + TG_B_STAGE);
     const int per = (p.halo ? 0 : TG_A_STAGE) + p.b_stage;
-    // a second store box per epilogue warp out of the ring's last 32 KB when at least 4 stages remain and the tile's mainloop
-    // is short (<= 48 k-steps, i.e. <= 96 * BN tensor cycles): those launches wait on TMA-store drain, not on operands; the
-    // long-K launches hide their epilogue anyway and keep the deeper ring
-    int ksteps = 0;
-    for (int t = 0; t < p.num_taps; ++t) ksteps += p.tap_kc[t];
-    p.ostg2 = (use_ostg2 && p.tma_out && ksteps <= 48 && (budget - TG_OSTG_BYTES) / per >= 4) ? 1 : 0;
-    if (p.ostg2) budget -= TG_OSTG_BYTES;
     p.stages = std::max(2, std::min(TG_MAX_STAGES, budget / per));
   }
   const CUtensorMap ta = encode_tmap(sa, dtype), tb = encode_tmap(sb, dtype);
@@ -634,7 +599,7 @@ void Engine::launch_gemm(Plan& P, const TmapSpec& sa, TmapSpec sb, const TapGemm
   }
   char shp[160];
   snprintf(shp, sizeof shp, "M=%.0f N=%d K=%.0f taps=%d BN=%d tiles=%lld grid=%d st=%d%s%s%s", m_valid, p.N, k_valid, p.num_taps, p.BN,
-           total_tiles, grid, p.stages, pair ? (p.halo ? " pair halo" : " pair") : "", p.tma_out ? (p.ostg2 ? " tma2" : " tma") : "",
+           total_tiles, grid, p.stages, pair ? (p.halo ? " pair halo" : " pair") : "", p.tma_out ? " tma" : "",
            (p.gn_part && p.tma_out) ? " gn" : "");
   // TMA-store epilogue: the output tensor map has the tile's row dims (extents = logical extents, so ragged edges are clipped
   // by the hardware) and a box of 64 columns x the 32 rows one epilogue warp owns
@@ -696,16 +661,6 @@ static void fill_strides(TmapSpec& s) {
 }
 
 Act Engine::conv(Plan& P, const Act& x, const PW& w, const ConvOpts& o_in) {
-  // A 3x3 conv's identity residual becomes one more K-slab (second source x identity weights): exact (bf16 * 1.0 accumulated
-  // in fp32) and it rides the TMA pipeline instead of latency-bound epilogue loads (+1/9 MMA work; r01: 0.85 -> see profiles)
-  if (use_idres && o_in.res && !o_in.x2 && o_in.ksize == 3 && o_in.stride == 1 && o_in.subpixel_phase < 0 && !o_in.out_fp32 &&
-      o_in.act != TG_ACT_GEGLU && o_in.res->C == w.rows && w.rows % 8 == 0 && w.rows <= 256 /* wider layers are MMA-bound */ && o_in.res->N == x.N && o_in.res->H == x.H &&
-      o_in.res->W == x.W) {
-    ConvOpts o2 = o_in;
-    const PW ident = prep_identity(w.rows);
-    o2.x2 = o_in.res; o2.w2 = &ident; o2.res = nullptr; o2.x2_identity = true;
-    return conv(P, x, w, o2);
-  }
   if (o_in.stride == 2 && ((x.H | x.W) & 1)) {
     // odd-sized map (latent of an image that is a multiple of 8 but not of 64): the right / bottom zero padding is materialised
     // once so that the 5-D parity view stays a plain box; Ho = ceil(H/2) as F.conv2d(stride=2, padding=1) gives
@@ -739,12 +694,7 @@ Act Engine::conv(Plan& P, const Act& x, const PW& w, const ConvOpts& o_in) {
   int tw, th, tn;
   const long long ldo = o.to_io_out_nchw ? 0 : out.ld;
   // halo mode (CTA-pair kernel): 8 x 16 output tiles whose nine taps share one halo tile per k-chunk
-#ifdef I2IT_HALO_X2
-  const bool halo_x2_ok = true;      // experimental build: the second-source taps ride a small A ring next to the halo stages
-#else
-  const bool halo_x2_ok = !o.x2;
-#endif
-  const bool want_halo = use_halo && use_pair && o.stride == 1 && k == 3 && !sub && halo_x2_ok && !o.to_io_out_nchw && x.H >= 16 &&
+  const bool want_halo = use_halo && use_pair && o.stride == 1 && k == 3 && !sub && !o.x2 && !o.to_io_out_nchw && x.H >= 16 &&
                          x.W >= 8 && x.C % 64 == 0;
   if (o.stride == 1) {
     tw = (x.H == 1) ? std::min(128, pow2ceil(x.W)) : std::min(o.to_io_out_nchw ? 32 : 16, pow2ceil(x.W));
@@ -956,7 +906,7 @@ Act Engine::conv(Plan& P, const Act& x, const PW& w, const ConvOpts& o_in) {
     p.tap_src[t2] = 1;
     p.tap_kc[t2] = ceil_div(o.x2->C, 64);
     p.num_taps = taps + 1;
-    k2 = o.x2_identity ? 0 : o.w2->cin;
+    k2 = o.w2->cin;
   }
   {
     const double m_valid = 1.0 * x.N * Ho * Wo, k_valid = 1.0 * taps * w.cin + k2;
@@ -1012,11 +962,9 @@ Act Engine::group_norm(Plan& P, const Act& x, const NormW& nw, float eps, bool s
   I2IT_CHECK(x.C == nw.C && x.C % 32 == 0 && x.C % 8 == 0, "group_norm: bad channel count " + std::to_string(x.C));
   const int C = x.C, HW = x.H * x.W, cg = C / 32, vecs = C / 8;
   I2IT_CHECK(vecs <= 1024, "group_norm: too many channels");
-  // tuning knobs (plan-build time): threads per CTA and CTAs per image
-  static const int env_thr = std::getenv("I2IT_GN_THREADS") ? atoi(std::getenv("I2IT_GN_THREADS")) : 128;   // measured best (r01 sweep)
-  static const int env_chunks = std::getenv("I2IT_GN_CHUNKS") ? atoi(std::getenv("I2IT_GN_CHUNKS")) : 512;
-  const int rows = std::max(1, std::min(1024, env_thr) / vecs), threads = vecs * rows;
-  const int chunks = std::max(1, std::min(env_chunks, ceil_div(HW, rows * 4)));
+  // about 128 threads per CTA and at most 512 CTAs per image: the best of the r01 sweep
+  const int rows = std::max(1, 128 / vecs), threads = vecs * rows;
+  const int chunks = std::max(1, std::min(512, ceil_div(HW, rows * 4)));
   // statistics pass over the tensor (no epilogue partials available): at most 64 chunk partials per image
   const int schunks = std::min(chunks, 64), spix = ceil_div(HW, schunks);
   const int pix = ceil_div(HW, chunks);
@@ -1166,7 +1114,7 @@ Act Engine::vt_proj(Plan& P, const Act& x, int B, int ntok, const PW& wv) {
 
 Act Engine::attention(Plan& P, const Act& q, const Act& k, const Act& vt, int B, int Nq, int Nk, int heads, int d,
                       int kv_batch) {
-  if (d == FA_D && use_flash) return flash_attention(P, q, k, vt, B, Nq, Nk, heads, kv_batch);
+  if (d == FA_D) return flash_attention(P, q, k, vt, B, Nq, Nk, heads, kv_batch);
   I2IT_CHECK(d % 64 == 0 && (d <= 256 || d % 256 == 0), "attention: head dim must be a multiple of 64");
 
   I2IT_CHECK(kv_batch == B || kv_batch == 1, "attention: kv batch must be 1 or B");
@@ -1308,10 +1256,8 @@ Act Engine::flash_attention(Plan& P, const Act& q, const Act& k, const Act& vt, 
   const int grid = fp.q_tiles * heads * B, dt = dtype;
   char shp[96];
   snprintf(shp, sizeof shp, "B=%d h=%d Nq=%d Nk=%d d=%d", B, heads, Nq, Nk, d);
-  const bool v1 = flash_v1;
   add_op(P, [=](cudaStream_t st) {
-    if (v1) { DISPATCH_T(dt, (launch_k(flash_attn_v1_kernel<T>, dim3(grid), dim3(FA_THREADS), FA_SMEM, st, 0, tq, tk, tv, fp))); }
-    else { DISPATCH_T(dt, (launch_k(flash_attn_kernel<T>, dim3(grid), dim3(FA_THREADS), FA_SMEM, st, 0, tq, tk, tv, fp))); }
+    DISPATCH_T(dt, (launch_k(flash_attn_kernel<T>, dim3(grid), dim3(FA_THREADS), FA_SMEM, st, 0, tq, tk, tv, fp)));
   }, "flash_attn", 4.0 * B * heads * Nq * Nk * d, 2.0 * (2.0 * B * Nq * C + 2.0 * kv_batch * Nk * C), shp);
   return out;
 }
@@ -1331,7 +1277,6 @@ void Engine::set_text(const void* text, int text_batch, cudaStream_t st) {
   TextKV& T = *slot;
   T.plan.io.text = text;
   nvtxRangePushA("i2it:text_kv");
-  g_pdl.enabled = false; g_pdl.prev_is_kernel = false;
   for (auto& op : T.plan.ops) op(st);
   nvtxRangePop();
   I2IT_CUDA(cudaGetLastError());
@@ -1396,7 +1341,6 @@ void Engine::encode_text(const int* tokens, int batch, void* out, cudaStream_t s
   P.io.x = tokens;
   P.io.out = out;
   nvtxRangePushA("i2it:clip_text_encoder");
-  g_pdl.enabled = false; g_pdl.prev_is_kernel = false;
   for (auto& op : P.ops) op(st);
   nvtxRangePop();
   I2IT_CUDA(cudaGetLastError());
@@ -1430,7 +1374,6 @@ void Engine::forward(const IO& io_in, int B, int H, int W, int direction, int te
       if (P->graphs.size() >= 8) { cudaGraphExecDestroy(P->graphs.front().second); P->graphs.erase(P->graphs.begin()); }
       cudaGraph_t g = nullptr;
       I2IT_CUDA(cudaStreamBeginCapture(gstream_, cudaStreamCaptureModeThreadLocal));
-      g_pdl.enabled = use_pdl; g_pdl.prev_is_kernel = false;
       for (auto& op : P->ops) op(gstream_);
       I2IT_CUDA(cudaStreamEndCapture(gstream_, &g));
       I2IT_CUDA(cudaGraphInstantiate(&ge, g, 0));
@@ -1443,7 +1386,6 @@ void Engine::forward(const IO& io_in, int B, int H, int W, int direction, int te
     I2IT_CUDA(cudaEventRecord(ev_out_, gstream_));
     I2IT_CUDA(cudaStreamWaitEvent(st, ev_out_, 0));
   } else {
-    g_pdl.enabled = use_pdl; g_pdl.prev_is_kernel = false;
     size_t next_range = 0;
     bool open = false;
     for (size_t i = 0; i < P->ops.size(); ++i) {
@@ -1501,7 +1443,6 @@ std::string Engine::profile_json(int reps, cudaStream_t st) {
   std::vector<double> ms(n, 0.0);
   for (int r = 0; r < reps; ++r) {
     I2IT_CUDA(cudaEventRecord(ev[0], st));
-    g_pdl.enabled = false;   // per-launch timing: full serialisation between kernels
     for (size_t i = 0; i < n; ++i) { P.ops[i](st); I2IT_CUDA(cudaEventRecord(ev[i + 1], st)); }
     I2IT_CUDA(cudaStreamSynchronize(st));
     for (size_t i = 0; i < n; ++i) { float t = 0; I2IT_CUDA(cudaEventElapsedTime(&t, ev[i], ev[i + 1])); ms[i] += t / reps; }

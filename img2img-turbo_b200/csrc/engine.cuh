@@ -14,7 +14,6 @@
 #include "prep.cuh"
 #include "tapgemm.cuh"
 #include "flash.cuh"
-#include "flash_v1.cuh"
 #include "tapgemm2.cuh"
 
 namespace i2it {
@@ -67,30 +66,21 @@ struct PW {                        // prepared (folded, re-laid-out) weight: [ta
   float* bias = nullptr;
   int rows = 0, cin = 0, cin_pad = 0, taps = 1;
 };
-// ---- kernel launch for plan ops: programmatic dependent launch (see pdl_sync in common.cuh) when the previous op of the
-// plan was also a kernel; `cluster` > 0 adds a (cluster,1,1) cluster dimension.  Executor state, one engine call per thread.
-struct PdlState { bool enabled = true; bool prev_is_kernel = false; };
-extern thread_local PdlState g_pdl;
+// ---- kernel launch for plan ops: `cluster` > 0 adds a (cluster,1,1) cluster dimension
 template <typename... KA, typename... A>
 inline void launch_k(void (*kern)(KA...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, int cluster, A&&... args) {
   cudaLaunchConfig_t cfg;
   std::memset(&cfg, 0, sizeof cfg);
   cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute at[2];
+  cudaLaunchAttribute at[1];
   unsigned n = 0;
   if (cluster > 0) {
     at[n].id = cudaLaunchAttributeClusterDimension;
     at[n].val.clusterDim.x = cluster; at[n].val.clusterDim.y = 1; at[n].val.clusterDim.z = 1;
     ++n;
   }
-  if (g_pdl.enabled && g_pdl.prev_is_kernel) {
-    at[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[n].val.programmaticStreamSerializationAllowed = 1;
-    ++n;
-  }
   cfg.attrs = at; cfg.numAttrs = n;
   cudaLaunchKernelEx(&cfg, kern, std::forward<A>(args)...);
-  g_pdl.prev_is_kernel = true;
 }
 
 struct NormW { const float* g = nullptr; const float* b = nullptr; int C = 0; };
@@ -141,7 +131,6 @@ struct ConvOpts {
   // second source folded into the same accumulator: out = conv(x) + conv1x1(x2)   (resnet conv_shortcut, decoder skip convs)
   const Act* x2 = nullptr;
   const PW* w2 = nullptr;
-  bool x2_identity = false;      // x2/w2 is the residual x identity trick: not algorithmic work (excluded from flop counts)
   int subpixel_phase = -1;       // >=0: this launch is parity phase (py*2+px) of a fused nearest-2x-upsample + 3x3 conv
   bool gn_out = false;           // the consumer of the output is a GroupNorm: take its statistics in this GEMM's epilogue
   std::shared_ptr<GnPart> gn_share;   // sub-pixel phases 1..3 add to the partial buffer phase 0 created
@@ -205,7 +194,6 @@ class Engine {
                 int kv_batch);
   Act flash_attention(Plan& P, const Act& q, const Act& k, const Act& vt, int B, int Nq, int Nk, int heads, int kv_batch,
                       bool causal = false);
-  bool use_flash = true, flash_v1 = false;
 
   // ---- weights ----
   bool has(const std::string& key) const;
@@ -214,7 +202,6 @@ class Engine {
           float scale = 1.f, const float* bias_add = nullptr);
   PW prep_twin(const std::string& pre, const std::string& cur, float r);
   PW prep_im2col3(const std::string& name);
-  PW prep_identity(int n);                                          // [n][n] identity as a 1x1 'weight'
   PW prep_subpixel(const std::string& name);                       // 16 pre-summed 2x2 taps for upsample2x+conv3x3
   Act conv_up2x(Plan& P, const Act& x, const PW& wsub, const Act* x2, const PW* w2, bool gn_out = false);                        // 3x3 conv over 3 channels as a K=32 single-tap GEMM
   NormW norm(const std::string& name);
@@ -248,9 +235,8 @@ class Engine {
   void launch_gemm(Plan& P, const TmapSpec& sa, TmapSpec sb, const TapGemmParams& p, bool out_from_io, const char* kind,
                    double k_valid, double bytes, const TmapSpec* sa2 = nullptr, const TmapSpec* sb2 = nullptr,
                    const TmapSpec* shalo = nullptr);
-  bool use_pair = true, use_halo = true, use_idres = true, use_pdl = false, trace_on = false, use_tmaout = true, use_gnepi = true, use_splitk = true, use_catfuse = true, use_ostg2 = true, use_lean = true, sync_each = false;
+  bool use_pair = true, use_halo = true, trace_on = false, use_tmaout = true, use_gnepi = true, use_splitk = true, use_lean = true, sync_each = false;
   bool tma_eligible(const TapGemmParams& p, bool out_from_io) const;
-  long long pair_min_tiles = 296;   // CTA-pair kernel from two waves of tiles upwards (tunable: I2IT_PAIR_MIN_TILES)
   std::string profile_json(int reps, cudaStream_t st);
   void dump_trace(Plan& P, cudaStream_t st);
   int pick_bn(long long m_tiles, int N, int step) const;   // step 64 / 128: BN restricted to multiples (TMA-store rounds)

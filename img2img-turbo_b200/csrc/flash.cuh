@@ -141,7 +141,6 @@ flash_attn_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  pdl_sync();   // prologue (barriers, TMEM, descriptor prefetch) overlaps the previous kernel's tail; no global access before here
   uint32_t tmem_base;
   asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
   const uint32_t tS0 = tmem_base, tPV = tmem_base + 128;   // S buffers at columns [0,64) and [64,128)

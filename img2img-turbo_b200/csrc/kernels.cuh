@@ -16,7 +16,6 @@ template <typename T>
 __global__ void gn_stats_kernel(const T* __restrict__ x, long long img_stride, int ld, int C, int HW, int cg,
                                 int pix_per_cta, float* __restrict__ partial /*[N][chunks][32][2]*/, int* __restrict__ counter,
                                 double inv_count, float eps, float* __restrict__ stats /*[N][32] (mean, rstd)*/) {
-  pdl_sync();
   extern __shared__ float s_acc[];   // [rows][2][C]: per-row partials, reduced in a fixed order (bit-reproducible)
   const int vecs = C >> 3;
   const int vx = threadIdx.x % vecs, vy = threadIdx.x / vecs, rows = blockDim.x / vecs;
@@ -99,7 +98,6 @@ __global__ void gn_stats_kernel(const T* __restrict__ x, long long img_stride, i
 static __global__ void gn_part_reduce_kernel(const float* __restrict__ part, int phases, int images, int slots, int per_row,
                                              int epg, int e_lanes /* pow2, <= 256 */, double2* __restrict__ scratch,
                                              int* __restrict__ counter, double inv_count, float eps, float* __restrict__ stats) {
-  pdl_sync();
   __shared__ double2 red[256];
   __shared__ double2 ent[640];                      // per_row <= 1280 / 2
   __shared__ int s_last;
@@ -171,7 +169,6 @@ template <typename T>
 __global__ void gn_apply_kernel(const T* __restrict__ x, long long ximg, int ldx, T* __restrict__ y, long long yimg,
                                 int ldy, int C, int HW, int cg, int pix_per_cta, const float* __restrict__ stats,
                                 const float* __restrict__ gamma, const float* __restrict__ beta, int silu) {
-  pdl_sync();
   const int vecs = C >> 3;
   const int vx = threadIdx.x % vecs, vy = threadIdx.x / vecs, rows = blockDim.x / vecs;
   const int n = blockIdx.y;
@@ -225,7 +222,6 @@ __global__ void gn_apply_kernel(const T* __restrict__ x, long long ximg, int ldx
 template <typename T>
 __global__ void layernorm_kernel(const T* __restrict__ x, int ldx, T* __restrict__ y, int ldy, int rows, int C,
                                  const float* __restrict__ gamma, const float* __restrict__ beta, float eps) {
-  pdl_sync();
   constexpr int MAXV = 5;   // C <= 1280
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= rows) return;
@@ -284,7 +280,6 @@ __global__ void layernorm_kernel(const T* __restrict__ x, int ldx, T* __restrict
 template <typename T, int TPR>
 __global__ void softmax_kernel(const float* __restrict__ s, long long lds, T* __restrict__ pr, long long ldp,
                                long long rows, int nk, int nk_pad) {
-  pdl_sync();
   constexpr int RPB = 128 / TPR;
   const long long row = static_cast<long long>(blockIdx.x) * RPB + threadIdx.x / TPR;
   const int tr = threadIdx.x % TPR;
@@ -333,7 +328,6 @@ __global__ void softmax_kernel(const float* __restrict__ s, long long lds, T* __
 // three strided passes over the fp32 logits (max, sum, write) — the logits of one row (<= a few tens of KB) stay in L1/L2.
 template <typename T>
 __global__ void softmax_long_kernel(const float* __restrict__ s, long long lds, T* __restrict__ pr, long long ldp, int nk, int nk_pad) {
-  pdl_sync();
   __shared__ float red[8];
   const long long row = blockIdx.x;
   const float* sr = s + row * lds;
@@ -367,7 +361,6 @@ __global__ void softmax_long_kernel(const float* __restrict__ s, long long lds, 
 template <typename T>
 __global__ void clip_embed_kernel(const int* __restrict__ ids, const float* __restrict__ tok, const float* __restrict__ pos,
                                   T* __restrict__ out, int C, int ntok, int vocab, long long total /* rows * C/8 */) {
-  pdl_sync();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= total) return;
   const int vecs = C >> 3;
@@ -389,7 +382,6 @@ __global__ void clip_embed_kernel(const int* __restrict__ ids, const float* __re
 // NCHW [B,3,H,W] (act dtype) -> NHWC8 (channels 3..7 zero): the 3-channel boundary of vae.encode.
 template <typename T>
 __global__ void pack_input_kernel(const T* __restrict__ x, T* __restrict__ y, int C, long long HW, long long total) {
-  pdl_sync();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;   // over B*HW pixels
   if (i >= total) return;
   const long long n = i / HW, p = i % HW;
@@ -406,7 +398,6 @@ __global__ void pack_input_kernel(const T* __restrict__ x, T* __restrict__ y, in
 // Turns encoder.conv_in (Cin=3: 16-byte TMA rows x 9 taps, TMA-request bound) into ONE K=32 GEMM tap with 64-byte rows.
 template <typename T>
 __global__ void pack_input_im2col_kernel(const T* __restrict__ x, T* __restrict__ y, int H, int W, long long total) {
-  pdl_sync();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;   // over B*H*W pixels
   if (i >= total) return;
   const long long HW = static_cast<long long>(H) * W;
@@ -445,7 +436,6 @@ __device__ __forceinline__ float u8_to_input(uint8_t q, int mode) {
 template <typename T>
 __global__ void pack_input_im2col_u8_kernel(const uint8_t* __restrict__ x /*[B,H,W,3]*/, T* __restrict__ y, int H, int W,
                                             long long total, int mode) {
-  pdl_sync();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;   // over B*H*W pixels
   if (i >= total) return;
   const long long HW = static_cast<long long>(H) * W;
@@ -475,7 +465,6 @@ __global__ void pack_input_im2col_u8_kernel(const uint8_t* __restrict__ x /*[B,H
 // .byte() (truncation).  NCHW [B,3,H,W] -> HWC uint8 [B,H,W,3].
 template <typename T>
 __global__ void nchw_to_u8hwc_kernel(const T* __restrict__ x, uint8_t* __restrict__ y, long long HW, long long total) {
-  pdl_sync();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;   // over B*H*W pixels
   if (i >= total) return;
   const long long n = i / HW, p = i % HW;
@@ -494,7 +483,6 @@ template <typename T>
 __global__ void latent_sample_kernel(const T* __restrict__ mom, int ldm, const T* __restrict__ eps_nchw,
                                      const T* __restrict__ noise_nchw, float r, float sf, T* __restrict__ z,
                                      long long HW, long long total) {
-  pdl_sync();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= total) return;
   const long long n = i / HW, p = i % HW;
@@ -529,7 +517,6 @@ template <typename T>
 __global__ void ddpm_step_kernel(const T* __restrict__ zin /*NHWC8*/, const T* __restrict__ pred, int ldp,
                                  float s1, float sa, float inv_sf, T* __restrict__ dec_in /*NHWC8*/,
                                  T* __restrict__ x0_nchw /*nullable*/, long long HW, long long total, int three_round) {
-  pdl_sync();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= total) return;
   const long long n = i / HW, p = i % HW;
@@ -558,7 +545,6 @@ __global__ void ddpm_step_kernel(const T* __restrict__ zin /*NHWC8*/, const T* _
 template <typename T>
 __global__ void upsample_nearest_kernel(const T* __restrict__ x, int ldx, T* __restrict__ y, int ldy, int H, int W, int Ho, int Wo,
                                         float sh, float sw, int C, long long total /* B*Ho*Wo*(C/8) */) {
-  pdl_sync();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= total) return;
   const int vecs = C >> 3;
@@ -577,7 +563,6 @@ __global__ void upsample_nearest_kernel(const T* __restrict__ x, int ldx, T* __r
 template <typename T>
 __global__ void pad_copy_kernel(const T* __restrict__ x, int ldx, T* __restrict__ y, int H, int W, int H2, int W2, int C,
                                 long long total /* B*H2*W2*(C/8) */) {
-  pdl_sync();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= total) return;
   const int vecs = C >> 3;
@@ -595,7 +580,6 @@ __global__ void pad_copy_kernel(const T* __restrict__ x, int ldx, T* __restrict_
 template <typename T>
 __global__ void splitk_reduce_kernel(const float* __restrict__ part, int S, long long split_stride, const float* __restrict__ bias,
                                      const T* __restrict__ res, int ldr, T* __restrict__ out, int ldo, int N, long long total /* rows*N/8 */) {
-  pdl_sync();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= total) return;
   const int vecs = N >> 3;
@@ -621,7 +605,6 @@ __global__ void splitk_reduce_kernel(const float* __restrict__ part, int S, long
 // strided 2-D copy of 16-byte vectors: rows x (C/8) vectors (torch.cat along channels)
 template <typename T>
 __global__ void copy2d_kernel(const T* __restrict__ x, int ldx, T* __restrict__ y, int ldy, int C, long long total) {
-  pdl_sync();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= total) return;
   const int vecs = C >> 3;

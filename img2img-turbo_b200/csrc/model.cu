@@ -235,7 +235,6 @@ void Engine::build_text_kv(TextKV& T) {
     Plan* plan = &P;
     add_op(P, [=](cudaStream_t st) {
       cudaMemcpyAsync(tp, plan->io.text, bytes, cudaMemcpyDeviceToDevice, st);
-      g_pdl.prev_is_kernel = false;
     });
   }
   for (const auto& p : xformer_prefixes()) {
@@ -267,23 +266,22 @@ Act Engine::build_unet(Plan& P, const Act& z, int text_batch, bool text_cached) 
     Plan* plan = &P;
     add_op(P, [=](cudaStream_t st) {
       cudaMemcpyAsync(tp, plan->io.text, bytes, cudaMemcpyDeviceToDevice, st);
-      g_pdl.prev_is_kernel = false;   // a copy node: the next kernel takes a full dependency
     });
   }
   // torch.cat([h, skip], dim=1) without copies: every skip connection is produced straight into the upper channel slice of
-  // the concat buffer its up-block resnet will read, and the running `h` into the lower slice (I2IT_NO_CATFUSE=1: copy kernels).
+  // the concat buffer its up-block resnet will read, and the running `h` into the lower slice.
   // Consumer q (pop order, 3 per up block) needs sC(q) channels of `h` in front of the skip.
   struct SkipSlot { Act cat, skip; int sC; };
   std::vector<SkipSlot> res;
   const int rch[4] = {ch[3], ch[2], ch[1], ch[0]};
   const int total_pushes = 12;                       // conv_in + 4 x 2 block outputs + 3 downsamplers
   int pushes = 0;
-  const bool fuse = use_catfuse;
   auto make_slot = [&](int N, int H, int W, int skipC) {
     const int q = total_pushes - 1 - pushes++, i = q / 3, j = q % 3;
     SkipSlot t;
     t.sC = (j == 0) ? (i == 0 ? ch[3] : rch[i - 1]) : rch[i];
-    if (fuse) { t.cat = alloc_act(P, N, H, W, t.sC + skipC); t.skip = t.cat.slice(t.sC, skipC); }
+    t.cat = alloc_act(P, N, H, W, t.sC + skipC);
+    t.skip = t.cat.slice(t.sC, skipC);
     return t;
   };
   auto push = [&](SkipSlot& t, const Act& produced) { t.skip = produced; res.push_back(t); };   // keeps the producer's GN partials
@@ -292,8 +290,7 @@ Act Engine::build_unet(Plan& P, const Act& z, int text_batch, bool text_cached) 
   Act s;
   {
     SkipSlot t = make_slot(z.N, z.H, z.W, ch[0]);
-    ConvOpts oc; oc.gn_out = true;
-    if (fuse) oc.out = &t.skip;
+    ConvOpts oc; oc.gn_out = true; oc.out = &t.skip;
     if (has(u + ".conv_in.conv_in_pretrained.weight"))
       s = conv(P, z, prep_twin(u + ".conv_in.conv_in_pretrained", u + ".conv_in.conv_in_curr", twin_r_), oc);
     else
@@ -306,15 +303,13 @@ Act Engine::build_unet(Plan& P, const Act& z, int text_batch, bool text_cached) 
       // who consumes the output decides whether the producing GEMM takes GroupNorm statistics: the transformer's GroupNorm
       // (i < 3), the next resnet's norm1 (j == 0, or the mid block after the last down block) — not the downsampler conv
       SkipSlot t = make_slot(s.N, s.H, s.W, ch[i]);
-      const Act* ov = fuse ? &t.skip : nullptr;
-      s = unet_resnet(P, blk + ".resnets." + std::to_string(j), s, true, i < 3 ? nullptr : ov);
-      if (i < 3) s = unet_xformer(P, blk + ".attentions." + std::to_string(j), s, heads[i], text_batch, j == 0, ov);
+      s = unet_resnet(P, blk + ".resnets." + std::to_string(j), s, true, i < 3 ? nullptr : &t.skip);
+      if (i < 3) s = unet_xformer(P, blk + ".attentions." + std::to_string(j), s, heads[i], text_batch, j == 0, &t.skip);
       push(t, s);
     }
     if (i < 3) {
       SkipSlot t = make_slot(s.N, (s.H + 1) / 2, (s.W + 1) / 2, ch[i]);
-      ConvOpts o; o.stride = 2; o.gn_out = true;
-      if (fuse) o.out = &t.skip;
+      ConvOpts o; o.stride = 2; o.gn_out = true; o.out = &t.skip;
       s = conv(P, s, prep(blk + ".downsamplers.0.conv", {blk + ".downsamplers.0.conv"}), o);
       push(t, s);
     }
@@ -323,9 +318,8 @@ Act Engine::build_unet(Plan& P, const Act& z, int text_batch, bool text_cached) 
   s = unet_resnet(P, u + ".mid_block.resnets.0", s, true);
   s = unet_xformer(P, u + ".mid_block.attentions.0", s, heads[3], text_batch, true);
   {
-    Act tgt;
-    if (fuse) tgt = h_target();
-    s = unet_resnet(P, u + ".mid_block.resnets.1", s, false, fuse ? &tgt : nullptr);   // -> concat (GroupNorm over the concatenation)
+    const Act tgt = h_target();
+    s = unet_resnet(P, u + ".mid_block.resnets.1", s, false, &tgt);   // -> concat (GroupNorm over the concatenation)
   }
   mark(P, "unet_mid", s);
   for (int i = 0; i < 4; ++i) {
@@ -334,22 +328,14 @@ Act Engine::build_unet(Plan& P, const Act& z, int text_batch, bool text_cached) 
     for (int j = 0; j < 3; ++j) {
       SkipSlot t = res.back();
       res.pop_back();
-      Act cat;
-      if (fuse) {
-        I2IT_CHECK(s.C == t.sC && s.p == t.cat.p && s.H == t.cat.H && s.W == t.cat.W, "unet: concat slot mismatch");
-        cat = t.cat;                                                   // both halves were written in place
-      } else {
-        cat = alloc_act(P, s.N, s.H, s.W, s.C + t.skip.C);             // torch.cat([h, skip], dim=1)
-        copy_channels(P, s, cat.slice(0, s.C));
-        copy_channels(P, t.skip, cat.slice(s.C, t.skip.C));
-      }
+      I2IT_CHECK(s.C == t.sC && s.p == t.cat.p && s.H == t.cat.H && s.W == t.cat.W, "unet: concat slot mismatch");
+      const Act cat = t.cat;                                           // both halves were written in place
       t = SkipSlot();
       const bool last = (i == 3 && j == 2);                            // the very last block feeds conv_norm_out directly
       // the block's output is the next concat's `h` unless an upsampler (j == 2, i < 3) or conv_norm_out (last) follows
       Act tgt;
-      const bool to_cat = fuse && j < 2;
-      if (to_cat) tgt = h_target();
-      const Act* ov = to_cat ? &tgt : nullptr;
+      if (j < 2) tgt = h_target();
+      const Act* ov = j < 2 ? &tgt : nullptr;
       s = unet_resnet(P, blk + ".resnets." + std::to_string(j), cat, i > 0, i > 0 ? nullptr : ov);
       if (i > 0) s = unet_xformer(P, blk + ".attentions." + std::to_string(j), s, hcount, text_batch, last, ov);
     }
@@ -358,9 +344,8 @@ Act Engine::build_unet(Plan& P, const Act& z, int text_batch, bool text_cached) 
       // — nearest to the spatial size of the next skip connection (e.g. 14 -> 27 columns for a 560x840 image)
       const SkipSlot& nxt = res.back();
       s = upsample_to(P, s, nxt.skip.H, nxt.skip.W);
-      Act tgt;
-      ConvOpts oc;
-      if (fuse) { tgt = h_target(); oc.out = &tgt; }
+      const Act tgt = h_target();
+      ConvOpts oc; oc.out = &tgt;
       s = conv(P, s, prep(blk + ".upsamplers.0.conv", {blk + ".upsamplers.0.conv"}), oc);
     }
   }

@@ -18,7 +18,6 @@ enum PrepMode : int {
   PREP_STORE = 0,      // out[tap][row_map(o)][cin_pad]                        (conv / linear weights, GEGLU interleave)
   PREP_SUBPIXEL = 1,   // out[phase*4 + ty*2+tx][o][cin_pad]: pre-summed 2x2 taps of nearest-2x + conv3x3
   PREP_IM2COL3 = 2,    // out[o][32], k = tap*3 + c                             (encoder.conv_in over 3 channels)
-  PREP_IDENTITY = 3,   // out[n][n] identity
   PREP_BIAS = 4,       // outf[row_map(o)] = c0*b[o] + c1*b1[o] + add[o]           (fp32; b1 = w1: TwinConv bias blend)
 };
 
@@ -30,7 +29,7 @@ struct PrepJob {
   const float* B[PREP_MAX_ADAPTERS];           // [cout][rank]
   float s[PREP_MAX_ADAPTERS];
   int rank[PREP_MAX_ADAPTERS];
-  void* out;                                   // 16-bit (modes 0-3) or fp32 (mode 4)
+  void* out;                                   // 16-bit (modes 0-2) or fp32 (mode 4)
   const float* bias; const float* bias_add;    // mode 4
   int mode, cout, cin, taps, cin_pad, rows_total, row_off, interleave_half;
   float scale;
@@ -105,8 +104,6 @@ __global__ void prep_jobs_kernel(const PrepJob* __restrict__ jobs, int njobs) {
       float v = 0.f;
       if (k < 27) v = prep_fold(j, o, k % 3, k / 3);
       reinterpret_cast<T*>(j.out)[i] = Elem<T>::from_f(v * j.scale);
-    } else if (j.mode == PREP_IDENTITY) {
-      reinterpret_cast<T*>(j.out)[i] = Elem<T>::from_f((i / j.cout) == (i % j.cout) ? 1.f : 0.f);
     } else {   // PREP_BIAS
       const int o = static_cast<int>(i);
       int orow = o;

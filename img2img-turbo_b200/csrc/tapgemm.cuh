@@ -25,20 +25,13 @@ namespace i2it {
 constexpr int TG_BM = 128;             // rows per tile (= TMEM lanes)
 constexpr int TG_BK = 64;              // K elements per stage (= 128 B = one swizzle atom)
 constexpr int TG_STAGES = 4;            // stages when the B tile is the full 32 KiB; smaller tiles get more (<= TG_MAX_STAGES)
-#ifndef I2IT_MAX_STAGES
-#define I2IT_MAX_STAGES 16          // `make STAGES8=1` builds the round-1 ring depth (8) into its own library for A/B runs
-#endif
-constexpr int TG_MAX_STAGES = I2IT_MAX_STAGES;   // small B tiles (BN <= 128) need more stages for the same lookahead in TIME
+constexpr int TG_MAX_STAGES = 16;      // small B tiles (BN <= 128) need more stages for the same lookahead in TIME
 constexpr int TG_MAX_TAPS = 16;
 constexpr int TG_A_STAGE = TG_BM * TG_BK * 2;    // 16 KiB
 constexpr int TG_B_STAGE = 256 * TG_BK * 2;      // 32 KiB (BN <= 256)
-#ifndef I2IT_EPI_WARPS
-#define I2IT_EPI_WARPS 8               // build-time: 8 (default) or 16 (`make EPI16=1`, experimental wide epilogue; see DESIGN §8)
-#endif
-constexpr int TG_EPI_WARPS = I2IT_EPI_WARPS;   // TG_EPI_GROUPS warps per TMEM lane quarter: they take the 32-column rounds in turn
+constexpr int TG_EPI_WARPS = 8;        // TG_EPI_GROUPS warps per TMEM lane quarter: they take the 32-column rounds in turn
 constexpr int TG_EPI_GROUPS = TG_EPI_WARPS / 4;
 constexpr int TG_EPI_RPW = 8 / TG_EPI_GROUPS;      // rounds per warp at BN = 256
-static_assert(TG_EPI_WARPS == 8, "epilogue warps: 8 (the 16-warp experiment of round 1 does not fit next to the 4 KB store boxes)");
 constexpr int TG_BAR_BYTES = 512;
 constexpr int TG_BIAS_BYTES = 2 * 256 * 4;       // per-tile bias slice, double-buffered like the accumulators
 // Epilogue store staging: each epilogue warp owns ONE TMA box = 32 rows x 64 output columns (128-byte rows, SWIZZLE_128B: the
@@ -78,7 +71,7 @@ struct TapGemmParams {
   int tap_kc[TG_MAX_TAPS];  // K chunks (of 64) for this tap
   int nprim;                // the first nprim taps share kchunks and are walked k-chunk-outer / tap-inner (same
                             // accumulation order in every kernel variant => bit-identical results); the rest follow
-  int stages, b_stage;      // smem ring: number of stages and bytes per B stage (sized to the actual tile, <= 8 stages)
+  int stages, b_stage;      // smem ring: number of stages and bytes per B stage (sized to the actual tile, <= TG_MAX_STAGES)
   int halo;                 // pair kernel only: 3x3 taps read shifted views of ONE halo tile per k-chunk
   int tap_a[TG_MAX_TAPS][5];
   int tap_b[TG_MAX_TAPS][4];
@@ -97,9 +90,6 @@ struct TapGemmParams {
   int act;
   int* err;               // device error word (watchdog)
   int tma_out;            // 1: 64-column rounds are staged in smem and stored by TMA (I2IT_NO_TMAOUT=1 -> 0: per-thread stores)
-  int ostg2;              // 1: every epilogue warp alternates between TWO store boxes (the second set lives in the last 32 KB of the
-                          // operand ring, which the host then sizes 32 KB smaller): a round no longer waits for the TMA store of
-                          // the previous round to drain its box (I2IT_NO_OSTG2=1 -> 0)
   // GroupNorm statistics of the OUTPUT tensor, taken from the staged (rounded) tile: per 32-row slot and per `gn_red` columns,
   // (sum, sum of squares) -> gn_part[(slot0 + m_tile*4 + quarter) * (N/gn_red) + col/gn_red][2]; nullptr = off
   float* gn_part;
@@ -174,7 +164,6 @@ __device__ __forceinline__ void tma_store_5d(const CUtensorMap* tm, uint32_t src
 }
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 // one lane of a fully converged warp (warp-uniform control flow keeps descriptors/addresses in uniform registers)
@@ -373,11 +362,10 @@ __device__ __forceinline__ void epilogue_chunk(const TapGemmParams& p, const uin
 template <typename T, bool LEAN>
 __device__ __forceinline__ void epilogue_tile(const TapGemmParams& p, const CUtensorMap* tmO, const TileCoord& c, int m_tile,
                                               int row, int warp, int j1, int j2, int j3, int j4, int acc, int aphase,
-                                              uint32_t tmem_base, float* s_bias, uint32_t ostg_base, uint32_t ostg2_base,
-                                              int& box_sel, uint32_t tfull_bar_addr, bool stage_bias, bool stamp = false) {
+                                              uint32_t tmem_base, float* s_bias, uint32_t ostg_base, uint32_t tfull_bar_addr,
+                                              bool stage_bias, bool stamp = false) {
   const int lane = threadIdx.x & 31;
-  // this warp's store box(es), 1024-byte aligned; with two boxes the warp alternates per round (box_sel persists across tiles)
-  const uint32_t ostg_w0 = ostg_base + warp * TG_OSTG_WARP, ostg_w1 = p.ostg2 ? ostg2_base + warp * TG_OSTG_WARP : ostg_w0;
+  const uint32_t ostg_warp = ostg_base + warp * TG_OSTG_WARP;   // this warp's store box, 1024-byte aligned
   const int grp = warp >> 2;                     // which of the two warps sharing this TMEM lane quarter
   const int g1 = c.t[0] * p.box[0] + j1, g2 = c.t[1] * p.box[1] + j2, g3 = c.t[2] * p.box[2] + j3,
             g4 = c.t[3] * p.box[3] + j4;
@@ -431,12 +419,10 @@ __device__ __forceinline__ void epilogue_tile(const TapGemmParams& p, const CUte
       if (r >= nrounds) break;                               // warp-uniform
       const int c0 = acols * r;                              // accumulator column of this round inside the tile
       if (n0 + c0 >= p.N) break;                             // whole round beyond N (last n-tile): nothing to store
-      // the previous TMA store out of this box must have finished READING it (two boxes: the store before the previous one)
-      const uint32_t ostg_warp = box_sel ? ostg_w1 : ostg_w0;
+      // the previous TMA store out of this box must have finished READING it
       const uint32_t my_row = ostg_warp + lane * 128;
-      if (lane == 0) { if (p.ostg2) bulk_wait_read1(); else bulk_wait_read0(); }
+      if (lane == 0) bulk_wait_read0();
       __syncwarp();
-      box_sel ^= p.ostg2;
       if (res_on) {
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
@@ -656,7 +642,6 @@ tapgemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   const uint32_t sA = base;
   const uint32_t sB = base + NS * TG_A_STAGE;
   const uint32_t ostg = base + TG_STAGES * (TG_A_STAGE + TG_B_STAGE);   // epilogue store boxes (1024-byte aligned)
-  const uint32_t ostg2 = ostg - TG_OSTG_BYTES;                          // optional second set: the ring's last 32 KB (p.ostg2)
   const uint32_t bars = ostg + TG_OSTG_BYTES;
   auto full_bar = [&](int s) { return bars + 8u * s; };
   auto empty_bar = [&](int s) { return bars + 8u * (TG_MAX_STAGES + s); };
@@ -690,7 +675,6 @@ tapgemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  pdl_sync();   // prologue (barriers, TMEM, descriptor prefetch) overlaps the previous kernel's tail; no global access before here
   if (threadIdx.x == 0) tg_stamp(p, 1);
   uint32_t tmem_base;
   asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
@@ -772,12 +756,12 @@ tapgemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const int j2 = rr % p.box[1]; rr /= p.box[1];
     const int j3 = rr % p.box[2];
     const int j4 = rr / p.box[2];
-    int iter = 0, box_sel = 0;
+    int iter = 0;
     for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++iter) {
       const int acc = iter & 1, aphase = (iter >> 1) & 1;
       const TileCoord c = decode_tile(p, tile);
-      epilogue_tile<T, LEAN>(p, &tmO, c, fast_div(tile, p.n_tiles, p.magic[0]), row, warp, j1, j2, j3, j4, acc, aphase, tmem_base, s_bias, ostg, ostg2,
-                       box_sel, tfull_bar(acc), p.n_tiles > 1 || iter < 2, iter == 0 && threadIdx.x == 0);
+      epilogue_tile<T, LEAN>(p, &tmO, c, fast_div(tile, p.n_tiles, p.magic[0]), row, warp, j1, j2, j3, j4, acc, aphase, tmem_base, s_bias, ostg,
+                       tfull_bar(acc), p.n_tiles > 1 || iter < 2, iter == 0 && threadIdx.x == 0);
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(tempty_bar(acc));

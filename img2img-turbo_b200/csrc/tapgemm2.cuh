@@ -21,19 +21,8 @@ constexpr int TG2_B_STAGE = 128 * TG_BK * 2;     // half of a BN<=256 weight til
 // view is "start + dy*2048 + dx*128" with SBO 2048 (swizzle phase from the absolute address, see umma_desc_halo).
 constexpr int TG2_HALO_W = 16, TG2_HALO_H = 18;
 constexpr int TG2_HALO_BYTES = TG2_HALO_H * TG2_HALO_W * TG_BK * 2;   // 36,864
-#ifdef I2IT_HALO_X2
-// experimental (`make HALOX2=1`): halo tiles also for convs with a second source (shortcut / identity / skip K-slab); the extra
-// taps' regular 128-row A boxes go through a small ring of their own next to two halo stages
-constexpr int TG2_HALO_STAGES = 2;
-constexpr int TG2_A2_STAGES = 2;
-#else
-#ifndef I2IT_HALO_STAGES
-#define I2IT_HALO_STAGES 2           // `make HALO3=1` builds a three-halo-stage library for A/B runs (fewer B stages)
-#endif
-constexpr int TG2_HALO_STAGES = I2IT_HALO_STAGES;   // two 36 KB halo tiles (each serves nine taps) leave room for the 32 KB of epilogue store boxes
-constexpr int TG2_A2_STAGES = 0;
-#endif
-constexpr int TG2_HALO_REGION = TG2_HALO_STAGES * TG2_HALO_BYTES + TG2_A2_STAGES * TG_A_STAGE;   // [halo stages][A2 stages]
+constexpr int TG2_HALO_STAGES = 2;   // two 36 KB halo tiles (each serves nine taps) leave room for the 32 KB of epilogue store boxes
+constexpr int TG2_HALO_REGION = TG2_HALO_STAGES * TG2_HALO_BYTES;
 constexpr int TG2_DATA_BYTES = TG2_STAGES * (TG_A_STAGE + TG2_B_STAGE);   // 192 KB; halo mode: [halo region][B stages in the rest]
 static_assert(TG2_HALO_REGION + 4 * TG2_B_STAGE <= TG2_DATA_BYTES, "halo region leaves fewer than four full B stages");
 constexpr int TG2_SMEM = TG2_DATA_BYTES + TG_BAR_BYTES + TG_BIAS_BYTES + TG_OSTG_BYTES + TG_ALIGN_PAD;
@@ -113,12 +102,11 @@ tapgemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     __trap();
   }
   // normal mode: [A stages][B stages]; halo mode: [halo stages][B stages]
-  const int NS = p.stages;                                  // host-chosen: B stage sized to the real half tile, <= 8 stages
+  const int NS = p.stages;                                  // host-chosen: B stage sized to the real half tile, <= TG_MAX_STAGES
   const uint32_t BST = static_cast<uint32_t>(p.b_stage);
   const uint32_t sA = base;
   const uint32_t sB = base + (p.halo ? TG2_HALO_REGION : NS * TG_A_STAGE);
   const uint32_t ostg = base + TG2_DATA_BYTES;                // epilogue store boxes (1024-byte aligned)
-  const uint32_t ostg2 = ostg - TG_OSTG_BYTES;                // optional second set: the ring's last 32 KB (p.ostg2)
   const uint32_t bars = ostg + TG_OSTG_BYTES;
   auto full_bar = [&](int s) { return bars + 8u * s; };
   auto empty_bar = [&](int s) { return bars + 8u * (TG_MAX_STAGES + s); };
@@ -127,11 +115,6 @@ tapgemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   const uint32_t tmem_slot = bars + 8u * (2 * TG_MAX_STAGES + 4);
   auto hfull_bar = [&](int s) { return bars + 8u * (2 * TG_MAX_STAGES + 6 + s); };
   auto hempty_bar = [&](int s) { return bars + 8u * (2 * TG_MAX_STAGES + 6 + TG2_HALO_STAGES + s); };
-#ifdef I2IT_HALO_X2
-  const uint32_t sA2 = base + TG2_HALO_STAGES * TG2_HALO_BYTES;
-  auto a2_empty_bar = [&](int s) { return bars + 8u * (2 * TG_MAX_STAGES + 6 + 2 * TG2_HALO_STAGES + s); };
-  static_assert(8 * (2 * TG_MAX_STAGES + 6 + 2 * TG2_HALO_STAGES + TG2_A2_STAGES) <= TG_BAR_BYTES, "barrier block too small");
-#endif
   float* const s_bias = reinterpret_cast<float*>(smem_raw + (bars - smem_u32(smem_raw)) + TG_BAR_BYTES);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -163,9 +146,6 @@ tapgemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     for (int s = 0; s < NS; ++s) { mbar_init(full_bar(s), 2); mbar_init(empty_bar(s), 1); }
     for (int a = 0; a < 2; ++a) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), 2 * TG_EPI_WARPS); }
     for (int s = 0; s < TG2_HALO_STAGES; ++s) { mbar_init(hfull_bar(s), 2); mbar_init(hempty_bar(s), 1); }
-#ifdef I2IT_HALO_X2
-    for (int s = 0; s < TG2_A2_STAGES; ++s) mbar_init(a2_empty_bar(s), 1);
-#endif
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmA)) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmB)) : "memory");
@@ -182,7 +162,6 @@ tapgemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  pdl_sync();   // prologue (barriers, TMEM, descriptor prefetch) overlaps the previous kernel's tail; no global access before here
   if (threadIdx.x == 0) tg_stamp(p, 1);
   uint32_t tmem_base;
   asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
@@ -194,9 +173,6 @@ tapgemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     // the N = 128 halo convs: this loop — per-step elect, parameter-table lookups — had become the critical path)
     if (elect_one()) {
     int stage = 0, phase = 0, hs = 0, hphase = 0;
-#ifdef I2IT_HALO_X2
-    int s2 = 0, a2phase = 0;
-#endif
     const uint32_t b_bytes = static_cast<uint32_t>(half_bn) * (TG_BK * 2);
     const uint32_t tx_bytes = 2u * (TG_A_STAGE + b_bytes);                                         // both CTAs' bytes
     for (int pt = cluster_id; pt < total_pairs; pt += num_clusters) {
@@ -237,27 +213,6 @@ tapgemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
             if (++stage == NS) { stage = 0; phase ^= 1; }
           }
         }
-#ifdef I2IT_HALO_X2
-        // second-source taps (shortcut / identity / skip K-slab): regular 128-row A boxes through the small A2 ring, B through
-        // the normal ring; both loads of a step complete on the B stage's full barrier
-        for (int t = p.nprim; t < p.num_taps; ++t)
-          for (int kc = 0; kc < p.tap_kc[t]; ++kc) {
-            const CUtensorMap* ta = p.tap_src[t] ? &tmA2 : &tmA;
-            const CUtensorMap* tb = p.tap_src[t] ? &tmB2 : &tmB;
-            mbar_wait(a2_empty_bar(s2), a2phase ^ 1, p.err, 26);
-            mbar_wait(empty_bar(stage), phase ^ 1, p.err, 21);
-            {
-              if (leader) mbar_expect_tx(full_bar(stage), tx_bytes);
-              else mbar_arrive_cluster(full_bar(stage), 0);
-              tma_load_5d_2sm(sA2 + s2 * TG_A_STAGE, ta, full_bar(stage), kc * TG_BK + p.tap_a[t][0], a1 + p.tap_a[t][1],
-                              a2 + p.tap_a[t][2], a3 + p.tap_a[t][3], a4 + p.tap_a[t][4]);
-              tma_load_5d_2sm(sB + stage * BST, tb, full_bar(stage), kc * TG_BK + p.tap_b[t][0], n0,
-                              b2 + p.tap_b[t][1], b3 + p.tap_b[t][2], b4 + p.tap_b[t][3]);
-            }
-            if (++stage == NS) { stage = 0; phase ^= 1; }
-            if (++s2 == TG2_A2_STAGES) { s2 = 0; a2phase ^= 1; }
-          }
-#endif
       } else {
         for (int kc = 0; kc < p.kchunks; ++kc)
           for (int t = 0; t < p.nprim; ++t) load_step(t, kc);
@@ -275,9 +230,6 @@ tapgemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     // short-MMA launches, see the halo branch); the other lanes wait at the warp barrier below.
     if (leader && elect_one()) {
       int stage = 0, phase = 0, iter = 0, hs = 0, hphase = 0;
-#ifdef I2IT_HALO_X2
-      int s2 = 0;
-#endif
       for (int pt = cluster_id; pt < total_pairs; pt += num_clusters, ++iter) {
         const int acc = iter & 1, aphase = (iter >> 1) & 1;
         mbar_wait(tempty_bar(acc), aphase ^ 1, p.err, 22);
@@ -288,7 +240,6 @@ tapgemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           // shifted by t/3 image rows = 2048 B and t%3 pixels = 128 B).  The r02h profile showed this single-thread loop, not
           // operands or TMEM, bounding the N = 128 convs: ~90 instructions (parameter-table lookups, R2UR moves) per 4 MMAs
           // of 64 cycles each = 55 % tensor pipe.
-          int s = 0;
           for (int kc = 0; kc < p.kchunks; ++kc) {
             mbar_wait(hfull_bar(hs), hphase, p.err, 25);
             const uint32_t a_base = sA + hs * TG2_HALO_BYTES;
@@ -309,28 +260,8 @@ tapgemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
               }
               if (++stage == NS) { stage = 0; phase ^= 1; }
             }
-            s += 9;
             if (++hs == TG2_HALO_STAGES) { hs = 0; hphase ^= 1; }
           }
-#ifdef I2IT_HALO_X2
-          for (int t = p.nprim; t < p.num_taps; ++t)
-            for (int kc = 0; kc < p.tap_kc[t]; ++kc, ++s) {
-              mbar_wait(full_bar(stage), phase, p.err, 23);
-              tc_fence_after();
-              {
-                const uint64_t adesc = umma_desc_sw128(sA2 + s2 * TG_A_STAGE);
-                const uint64_t bdesc = umma_desc_sw128(sB + stage * BST);
-#pragma unroll
-                for (int k = 0; k < TG_BK / 16; ++k)
-                  tc_mma_f16_2sm(d_tmem, adesc + 2 * k, bdesc + 2 * k, p.idesc, 1u);
-                tc_commit_2sm(empty_bar(stage));
-                tc_commit_2sm(a2_empty_bar(s2));
-                if (s == steps - 1) tc_commit_2sm(tfull_bar(acc));
-              }
-              if (++stage == NS) { stage = 0; phase ^= 1; }
-              if (++s2 == TG2_A2_STAGES) s2 = 0;
-            }
-#endif
         } else {
           for (int s = 0; s < steps; ++s) {
             mbar_wait(full_bar(stage), phase, p.err, 23);
@@ -361,12 +292,12 @@ tapgemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     const int j2 = rr % p.box[1]; rr /= p.box[1];
     const int j3 = rr % p.box[2];
     const int j4 = rr / p.box[2];
-    int iter = 0, box_sel = 0;
+    int iter = 0;
     for (int pt = cluster_id; pt < total_pairs; pt += num_clusters, ++iter) {
       const int acc = iter & 1, aphase = (iter >> 1) & 1;
       const TileCoord c = decode_pair(pt);
       epilogue_tile<T, LEAN>(p, &tmO, c, 2 * fast_div(pt, p.n_tiles, p.magic[0]) + static_cast<int>(rank), row, warp, j1, j2, j3, j4, acc, aphase,
-                       tmem_base, s_bias, ostg, ostg2, box_sel, tfull_bar(acc), p.n_tiles > 1 || iter < 2, iter == 0 && threadIdx.x == 0);
+                       tmem_base, s_bias, ostg, tfull_bar(acc), p.n_tiles > 1 || iter < 2, iter == 0 && threadIdx.x == 0);
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(tempty_bar(acc), 0);

@@ -215,7 +215,7 @@ def test_resolutions_that_are_multiples_of_8_not_64(hw):
 
 def test_runtime_switches_agree(monkeypatch):
     """Every A/B switch of the engine selects another hand-written CUDA variant of the same arithmetic: outputs agree, and bit
-    for bit where the variant only changes data movement (in-place concat, TMA vs per-thread stores with the statistics kernel)."""
+    for bit where the variant only changes data movement (lean epilogue, TMA vs per-thread stores with the statistics kernel)."""
     import weights as W
     cfg, dt = W.TINY, torch.bfloat16
     sd = W.make_state_dict("pix2pix", cfg, seed=0, perturb_norm=True)
@@ -223,9 +223,7 @@ def test_runtime_switches_agree(monkeypatch):
     args = (x.to(dt).cuda(), text[:1].to(dt).cuda(), eps.to(dt).cuda())
 
     def run(**env):
-        for k in ("I2IT_NO_CATFUSE", "I2IT_NO_TMAOUT", "I2IT_NO_GNEPI", "I2IT_NO_SPLITK", "I2IT_FLASH_V1", "I2IT_NO_IDRES", "I2IT_IDRES",
-                  "I2IT_NO_LEAN", "I2IT_NO_OSTG2",
-                  "I2IT_NO_HALO", "I2IT_NO_PAIR"):
+        for k in ("I2IT_NO_TMAOUT", "I2IT_NO_GNEPI", "I2IT_NO_SPLITK", "I2IT_NO_LEAN", "I2IT_NO_HALO", "I2IT_NO_PAIR"):
             monkeypatch.delenv(k, raising=False)
         for k, v in env.items():
             monkeypatch.setenv(k, v)
@@ -235,12 +233,9 @@ def test_runtime_switches_agree(monkeypatch):
         e.close()
         return y
     base = run()
-    assert torch.equal(base, run(I2IT_NO_CATFUSE="1"))
     assert torch.equal(base, run(I2IT_NO_LEAN="1"))            # the compile-time-stripped epilogue computes the same bits
-    assert torch.equal(base, run(I2IT_NO_OSTG2="1"))           # one or two store boxes: data movement only
     assert torch.equal(run(I2IT_NO_GNEPI="1"), run(I2IT_NO_GNEPI="1", I2IT_NO_TMAOUT="1"))
-    for env in ({"I2IT_NO_GNEPI": "1"}, {"I2IT_NO_SPLITK": "1"}, {"I2IT_FLASH_V1": "1"}, {"I2IT_IDRES": "1"},
-                {"I2IT_NO_HALO": "1"}, {"I2IT_NO_PAIR": "1"}):
+    for env in ({"I2IT_NO_GNEPI": "1"}, {"I2IT_NO_SPLITK": "1"}, {"I2IT_NO_HALO": "1"}, {"I2IT_NO_PAIR": "1"}):
         y = run(**env)
         d = (y.float() - base.float()).abs()
         # different summation orders of the fp32 statistics / K ranges flip last bits of bf16 activations (1 ulp at 1.0 = 7.8e-3),
